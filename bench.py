@@ -3,6 +3,7 @@
 
   python bench.py --gpus N --steps K --warmup W          our CUDA path (one process per GPU under torchrun)
   python bench.py --impl reference --steps K --warmup W  the reference's own SSE2 path on the host cores
+  python bench.py ... --dump-outputs DIR                  also write the records of every shape's last timed step (dump_outputs)
 
 Headline workload (BASELINE.json configs[2], SURVEY 8(d) "config 3", the shape north_star's scaling target is quoted on):
 100,000 synthetic 150 bp DNA reads x one 5 Mbp reference, DNA matrix 2/-2 (N = 0), gap open 3 / extend 1, score_size 2
@@ -29,6 +30,7 @@ import time
 
 import numpy as np
 
+sys.dont_write_bytecode = True          # the tree may be read-only: nothing is written there, not even __pycache__
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "tests"))
@@ -64,7 +66,13 @@ def parse():
     ap.add_argument("--dry-run-emu", action="store_true",
                     help="tests only: run the orchestration on the CPU emulator build of the kernels (tests/cuda_emu) with tiny shapes and "
                          "the gloo backend; the printed line is marked dry_run and its numbers mean nothing")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the records (and CIGAR words) the last timed step of every shape returned as "
+                         "DIR/<shape>_<field>.npy, float64 (see dump_outputs)")
+    args = ap.parse_args()
+    if args.steps < 1 or args.sub_steps < 1:
+        ap.error("--steps and --sub-steps must be at least 1")
+    return args
 
 
 def workload_name(n_reads):
@@ -242,8 +250,9 @@ def shard_of(W, cfg, D, rank, world):
     return D.shard_range(cells, rank, world)
 
 
-def run_shape(X, cfg, W, steps, warmup, e2e_reps, sampler=None):
-    """Time one shape.  Returns (stats dict on every rank, gathered records + pool on rank 0)."""
+def run_shape(X, cfg, W, steps, warmup, e2e_reps, sampler=None, dump=None):
+    """Time one shape.  Returns (stats dict on every rank, gathered records + pool on rank 0).  dump: called on rank 0 with
+    what the last timed step returned, before the end-to-end repetitions re-use its buffers."""
     import torch
     import torch.distributed as dist
     D, L, eng = X.D, X.L, X.eng
@@ -295,6 +304,8 @@ def run_shape(X, cfg, W, steps, warmup, e2e_reps, sampler=None):
         fill_launches += tm["fill_forward_launches"]
         overflows = tm["byte_overflows"]
     clocks = sampler.stop() if (sampler is not None and X.rank == 0) else None
+    if dump is not None and X.rank == 0:
+        dump(got)
     tt = torch.tensor([acc["total_ms"], wall * 1e3, acc["fill_forward_ms"], acc["resolve_ms"], acc["fill_reverse_ms"], acc["traceback_ms"]],
                       dtype=torch.float64, device=dev)
     cnt = torch.tensor([launches, fill_launches, overflows], dtype=torch.int64, device=dev)
@@ -332,6 +343,37 @@ def run_shape(X, cfg, W, steps, warmup, e2e_reps, sampler=None):
              "h2d_rank0": h2d, "d2h_rank0": int(36 * n_pairs_rank + (4 * len(got[1]) if (got and got[1] is not None and X.world == 1) else 0)),
              "pairs": n_q_all * n_r, "shard": [lo, hi], "clocks": clocks, "steps": steps, "warmup": warmup}
     return stats, got
+
+
+DUMP_FIELDS = ("score1", "score2", "ref_begin1", "ref_end1", "read_begin1", "read_end1", "ref_end2", "flag", "status", "cigar_len")
+DUMP_PAIRS = 1 << 18                     # records per shape at most: 10 fields x 8 bytes x 262,144 = 21 MB
+DUMP_LIMIT = 64 << 20
+
+
+def dump_outputs(out_dir, shape, got):
+    """rank 0: the records of the last timed step, one float64 array per field (DIR/<shape>_<field>.npy, pair order), and the
+    CIGAR words of those pairs concatenated in pair order (DIR/<shape>_cigar.npy, written only when there are any: shapes run
+    with flag 0 return no CIGAR; cigar_len splits them).  A shape with more
+    than DUMP_PAIRS pairs is written as a fixed, seeded sample of them, whose pair indices go to DIR/<shape>_pair_index.npy.
+    The inputs are seeded too, so two builds run with the same arguments can be compared array by array.  Returns the bytes
+    written."""
+    recs, pool = got
+    pool = np.zeros(0, np.uint32) if pool is None else np.asarray(pool)
+    idx = np.arange(len(recs))
+    if len(recs) > DUMP_PAIRS:
+        idx = np.sort(np.random.default_rng(0).choice(len(recs), DUMP_PAIRS, replace=False))
+    arrays = {f: recs[f][idx].astype(np.float64) for f in DUMP_FIELDS}
+    if len(idx) != len(recs):
+        arrays["pair_index"] = idx.astype(np.float64)
+    offs, lens = recs["cigar_off"][idx].astype(np.int64), recs["cigar_len"][idx].astype(np.int64)
+    lens = np.where(offs < 0, 0, lens)
+    starts = np.concatenate([[0], np.cumsum(lens)])
+    if starts[-1] > 0:
+        arrays["cigar"] = pool[np.repeat(offs - starts[:-1], lens) + np.arange(starts[-1])].astype(np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, "%s_%s.npy" % (shape, name)), a)
+    return sum(a.nbytes for a in arrays.values())
 
 
 def parity_check(W, got, n_check, n_r):
@@ -429,7 +471,14 @@ def main():
     tiny = dict(ref_len=2000, read_len=60) if X.emu else {}
     W3 = C.config_workload(3, n_reads=args.reads, **tiny)
     sampler = {"smi": ClockSampler, "nvml": NvmlSampler}[args.clock_sampler](X.local)
-    st3, got3 = run_shape(X, 3, W3, args.steps, args.warmup, args.e2e_reps, sampler)
+    dumped = []
+
+    def dumper(shape):
+        if args.dump_outputs:
+            return lambda got: dumped.append(dump_outputs(args.dump_outputs, shape, got))
+        return None
+
+    st3, got3 = run_shape(X, 3, W3, args.steps, args.warmup, args.e2e_reps, sampler, dumper("config3"))
     line = None
     if rank0:
         hbm_peak, peak_src = peaks()
@@ -484,7 +533,7 @@ def main():
     subs = {}
     if 2 in only:
         W = C.config_workload(2, **(dict(n_reads=4, **tiny) if X.emu else {}))
-        st, got = run_shape(X, 2, W, max(args.sub_steps, 3), 3, args.e2e_reps)
+        st, got = run_shape(X, 2, W, max(args.sub_steps, 3), 3, args.e2e_reps, dump=dumper("config2"))
         if rank0:
             o = sub_result(st, X.world, "config2", "1,000 x 150 bp reads vs 5 Mbp, byte-score path, flag 0 (strong: reads split over the GPUs)")
             ref_len = len(W["refs"][0])
@@ -500,7 +549,7 @@ def main():
             subs["config2"] = o
     if 4 in only:
         W = C.config_workload(4, n_queries=args.c4_queries, n_targets=args.c4_targets)
-        st, got = run_shape(X, 4, W, args.sub_steps, 2, args.e2e_reps)
+        st, got = run_shape(X, 4, W, args.sub_steps, 2, args.e2e_reps, dump=dumper("config4"))
         if rank0:
             o = sub_result(st, X.world, "config4", "protein BLOSUM50, word-score path, flag 0: a %d-query slice of the 10,000 x 300 aa queries x all %d x 400 aa targets "
                            "(queries split over the GPUs, targets replicated; the full grid would return 18 GB of records)" % (args.c4_queries, args.c4_targets))
@@ -513,7 +562,7 @@ def main():
         del got
     if 5 in only:
         W = C.config_workload(5, **(dict(n_reads=3, ref_len=1500, read_len=330) if X.emu else {}))
-        st, got = run_shape(X, 5, W, args.sub_steps, 2, args.e2e_reps)
+        st, got = run_shape(X, 5, W, args.sub_steps, 2, args.e2e_reps, dump=dumper("config5"))
         if rank0:
             o = sub_result(st, X.world, "config5", "1,000 x 10 kbp reads vs 100 kbp, byte pass overflows -> word path, flag 2 (begin search + banded traceback, "
                            "CIGARs gathered in two phases: lengths, then payload)")
@@ -530,6 +579,9 @@ def main():
         bad = line["parity"]["config3"]["mismatches"] + sum(s["parity"]["mismatches"] for s in subs.values())
         line["parity_checked"] = line["parity"]["config3"]["parity_checked"] + sum(s["parity"]["parity_checked"] for s in subs.values())
         line["mismatches"] = bad
+        if args.dump_outputs:
+            assert sum(dumped) <= DUMP_LIMIT, dumped
+            line["dumped_bytes"] = sum(dumped)
         print(json.dumps(line))
     X.eng.close()
     if X.world > 1:

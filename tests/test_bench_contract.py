@@ -50,9 +50,25 @@ def _check_b200_line(d, world):
         assert d["cpu_baseline"]["kind"] in ("reference", "port") and "cpu_baseline" in d["config4"]
 
 
-def test_b200_arm_dry_run_on_emulator_world1():
-    out = subprocess.run([sys.executable, os.path.join(C.ROOT, "bench.py"), "--gpus", "1"] + DRY, capture_output=True, text=True, timeout=900)
-    _check_b200_line(_one_line(out), 1)
+def test_b200_arm_dry_run_on_emulator_world1(tmp_path):
+    out = subprocess.run([sys.executable, os.path.join(C.ROOT, "bench.py"), "--gpus", "1", "--dump-outputs", str(tmp_path)] + DRY,
+                         capture_output=True, text=True, timeout=900)
+    d = _one_line(out)
+    _check_b200_line(d, 1)
+    import numpy as np
+    for shape, pairs in (("config3", 7), ("config2", 4), ("config4", 15), ("config5", 3)):
+        a = {f: np.load(tmp_path / ("%s_%s.npy" % (shape, f))) for f in ("score1", "ref_end1", "status", "cigar_len")}
+        assert len(a["score1"]) == len(a["ref_end1"]) == pairs and (a["score1"] > 0).any()
+        cigar = tmp_path / ("%s_cigar.npy" % shape)
+        assert cigar.exists() == (shape == "config5")          # flag 2: CIGARs; the other shapes run flag 0
+        if cigar.exists():
+            a["cigar"] = np.load(cigar)
+            assert len(a["cigar"]) == a["cigar_len"].sum() > 0
+        assert all(x.dtype == np.float64 for x in a.values())
+    files = list(tmp_path.iterdir())
+    assert all(np.load(p).size > 0 for p in files)
+    total = sum(os.path.getsize(p) for p in files)
+    assert 0 < d["dumped_bytes"] <= total <= 64 << 20
 
 
 def test_b200_arm_dry_run_on_emulator_torchrun_world2():

@@ -409,47 +409,59 @@ def test_emulated_align_batch_c_entry(oracle, capfd):
     eng.close()
 
 
-@pytest.mark.skipif(not os.path.exists("/root/reference/src/pyssw.py"), reason="reference tree not present (build container only)")
+def _prebuilt(name):
+    """A program of the reference that build() puts in oracle/_ref (made where the reference's source is at hand)."""
+    path = os.path.join(C.ORACLE_DIR, "_ref", name)
+    if not os.path.exists(path):
+        pytest.skip("oracle/_ref/%s not built: the reference's source was not at hand when the checkers were built" % name)
+    return path
+
+
+def _consumer_files(tmp_path):
+    """Writes the demo inputs frozen in consumer_outputs.json into tmp_path; returns the frozen runs."""
+    with open(os.path.join(C.GOLDEN, "consumer_outputs.json")) as f:
+        G = json.load(f)
+    for name, text in G["files"].items():
+        (tmp_path / name).write_text(text)
+    return G
+
+
 def test_reference_python_driver_unmodified(tmp_path):
     """The reference's own pyssw.py + ssw_lib.py (ctypes) load a library by the name libssw.so: given the emulator build
     of our sources they print what they print with the reference's ssw.c (the ctypes struct mirrors stay compatible)."""
+    pyssw = _prebuilt("pyssw.py")
     subprocess.run(["make", "-s", "-C", EMU_DIR], check=True)
     if not C.have_ref():
         pytest.skip("compiled reference not available")
+    _consumer_files(tmp_path)
     outs = []
     for name, lib in (("ours", os.path.join(EMU_DIR, "libssw_emu.so")), ("ref", C.LIB_REF)):
         d = tmp_path / name
         d.mkdir()
         os.symlink(lib, d / "libssw.so")
-        r = subprocess.run([sys.executable, "/root/reference/src/pyssw.py", "-l", str(d), "-c", "/root/reference/demo/r1.fa",
-                            "/root/reference/demo/r1_query.fq"], capture_output=True, text=True, timeout=300, cwd=str(tmp_path))
+        r = subprocess.run([sys.executable, pyssw, "-l", str(d), "-c", "r1.fa", "r1_query.fq"], capture_output=True, text=True, timeout=300,
+                           cwd=str(tmp_path), env=dict(os.environ, PYTHONDONTWRITEBYTECODE="1"))
         assert r.returncode == 0, r.stderr[-500:]
         outs.append("\n".join(l for l in r.stdout.splitlines() if not l.startswith("CPU time")))
     assert outs[0] == outs[1] and "optimal_alignment_score: 52" in outs[0]
 
 
-@pytest.mark.skipif(not os.path.exists("/root/reference/src/main.c"), reason="reference tree not present (build container only)")
 def test_reference_c_consumers_unmodified_on_emulator_build(tmp_path):
     """CPU replica of test_gpu_parity.py::test_unmodified_reference_consumers_on_our_library: the reference's ssw_test,
-    example_c and example_cpp, compiled unmodified against the emulator build of our sources, reproduce the frozen outputs."""
+    example_c and example_cpp, built unmodified against libssw.so (oracle/_ref/*_b200), run over the emulator build of our
+    sources (found through LD_LIBRARY_PATH, which comes before their run path) and reproduce the frozen outputs."""
+    exe = {name: _prebuilt(name + "_b200") for name in ("ssw_test", "example_c", "example_cpp")}
     subprocess.run(["make", "-s", "-C", EMU_DIR], check=True)
-    ref = "/root/reference/src"
-    link = ["-L" + EMU_DIR, "-l:libssw_emu.so", "-Wl,-rpath," + EMU_DIR, "-lm", "-lz"]
-    exe = {}
-    for name, cmd in (("ssw_test", ["gcc", "-O2", "-o", str(tmp_path / "ssw_test"), ref + "/main.c"] + link),
-                      ("example_c", ["gcc", "-O2", "-o", str(tmp_path / "example_c"), ref + "/example.c"] + link),
-                      ("example_cpp", ["g++", "-O2", "-o", str(tmp_path / "example_cpp"), ref + "/example.cpp", ref + "/ssw_cpp.cpp"] + link)):
-        subprocess.run(cmd, check=True)
-        exe[name] = str(tmp_path / name)
-    with open(os.path.join(C.GOLDEN, "consumer_outputs.json")) as f:
-        G = json.load(f)
-    for name, text in G["files"].items():
-        (tmp_path / name).write_text(text)
+    lib = tmp_path / "lib"
+    lib.mkdir()
+    os.symlink(os.path.join(EMU_DIR, "libssw_emu.so"), lib / "libssw.so")
+    env = dict(os.environ, LD_LIBRARY_PATH=os.pathsep.join(p for p in (str(lib), os.environ.get("LD_LIBRARY_PATH")) if p))
+    G = _consumer_files(tmp_path)
     n = 0
     for run in G["runs"]:
         if "1k.fa" in run["args"]:
             continue                       # 100 reads per run: minutes on the emulator; the GPU suite runs them
-        out = subprocess.run([exe[run["exe"]]] + run["args"], capture_output=True, text=True, timeout=600, cwd=str(tmp_path))
+        out = subprocess.run([exe[run["exe"]]] + run["args"], capture_output=True, text=True, timeout=600, cwd=str(tmp_path), env=env)
         got = "\n".join(l for l in out.stdout.splitlines() if not l.startswith("CPU time"))
         assert got == run["stdout"], (run["exe"], run["args"])
         n += 1
